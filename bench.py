@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- predict_rank throughput of the B200-native hot path (BASELINE.json metric), one JSON line on stdout.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json north_star / SURVEY.md 8d, "C5 at 1M x 1M"): predict_rank top-10 over 1M users x 1M items,
 n_components = 128, indicator-regime sparse features (identity + 3 random tags per row, F = 1.2 R, ~4 nnz/row),
@@ -290,6 +290,28 @@ def oracle_topk_rows(uf, itf, wu, wi, bu, bi, rows, k, item_repr=None, item_bias
     return out, item_repr, item_bias
 
 
+DUMP_BYTES = 48 << 20      # --dump-outputs budget: a seeded row sample keeps larger results under 64 MB
+
+
+def dump_topk(out_dir, top, first_user):
+    """Writes the top-k a caller of the timed path receives (item ids, scores) for a fixed, seeded sample of its user
+    rows (all rows when they fit DUMP_BYTES), with the global user id of every row.  Ids are stored as float64 (exact
+    for any int32), scores as float32."""
+    import torch
+    n_users, k = top.items.shape
+    n_rows = min(n_users, DUMP_BYTES // (8 + k * (8 + 4)))
+    rows = np.arange(n_users) if n_rows == n_users else \
+        np.sort(np.random.default_rng(0).choice(n_users, n_rows, replace=False))
+    idx = torch.from_numpy(rows).to(top.items.device)
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'user_ids': (rows + first_user).astype(np.float64),
+              'topk_items': top.items[idx].cpu().numpy().astype(np.float64),
+              'topk_scores': top.scores[idx].cpu().numpy().astype(np.float32)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), arr)
+    log('[bench] wrote %s (%d of %d user rows, top-%d)' % (', '.join(n + '.npy' for n in arrays), n_rows, n_users, k))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -432,6 +454,8 @@ def run_b200(args):
     ms_total = start.elapsed_time(end)
     clocks = (sampler.stop() if not args.no_clocks else {'sm_mhz': None, 'reasons': ['sampling disabled']}) \
         if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_topk(args.dump_outputs, out, u_lo)
     t = torch.tensor([ms_total], device=dev, dtype=torch.float64)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -618,7 +642,6 @@ def run_extras(args):
         a = copy.copy(args)
         for key, val in over.items():
             setattr(a, key, val)
-        a.steps, a.warmup = 3, 2
         try:
             extras[name] = fn(a, emit=False)
         except Exception as exc:      # a secondary line must not take the headline down
@@ -965,7 +988,14 @@ def main():
     ap.add_argument('--n-sampled', type=int, default=64, help='--workload train: n_sampled_items')
     ap.add_argument('--train-dtype', default='bf16', choices=['bf16', 'f32'], help='--workload train: representations')
     ap.add_argument('--train-cpu-users', type=int, default=20000, help='--workload train: users of the CPU oracle sample')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the top-k of the last step (a seeded sample of its user rows) '
+                         'as DIR/<name>.npy, for output-for-output comparison of two builds')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and (args.workload != 'topk' or args.impl != 'b200'):
+        ap.error('--dump-outputs writes the top-k of --workload topk --impl b200')
     if args.workload == 'dense':
         run_dense(args)
     elif args.workload == 'ranks':

@@ -1,43 +1,26 @@
-"""Drop-in check: the REFERENCE'S OWN, unmodified test files run against this package through compat/ (a `tensorrec`
-alias package, a torch-backed `tensorflow` stand-in for the handful of TF names its tests use, and a
-`nose_parameterized` shim).  Only the tests that need no device run here -- everything that reaches predict /
-predict_rank requires a CUDA device (no CPU fallback), and /root/reference does not exist on the GPU box, so those are
-covered by this repo's own GPU tests, which restate them (tests/test_api_gpu.py, tests/test_kernels_gpu.py).
-
-Skipped when the reference checkout is absent."""
+"""Drop-in check: the cases of the REFERENCE'S OWN test suite that need no device, restated in tests/reference_cases.py,
+run against this package through compat/ (a `tensorrec` alias package, a torch-backed `tensorflow` stand-in for the
+handful of TF names those tests use, and a `nose_parameterized` shim) in a process of their own.  Every case the
+reference's unmodified test files passed with (tests/golden/reference_suite_cases.json) must pass.  The reference tests
+that reach predict / predict_rank need a CUDA device (no CPU fallback) and are restated by this repo's own GPU tests
+(tests/test_api_gpu.py, tests/test_kernels_gpu.py)."""
+import json
 import os
-import re
 import subprocess
 import sys
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFERENCE_TESTS = '/root/reference/test'
-
-# (file, -k expression or None, number of tests that must pass)
-CPU_RUNNABLE = [
-    ('test_util.py', None, 1),
-    ('test_loss_graphs.py', None, 8),                       # fit with every loss graph
-    ('test_representation_graphs.py', None, 8),             # nose_parameterized fits + the two dimension errors
-    ('test_tensorrec.py::TensorRecTestCase', None, 17),     # constructor checks, fit variants, datasets, TFRecords
-    ('test_readme.py', 'custom', 2),                        # user-defined representation / loss graphs on `tf` names
-    ('test_prediction_graphs.py', 'serial or PredictionGraphsTestCase', 5),
-    ('test_recommendation_graphs.py', 'project_biases or split or serial or densify', 4),
-]
+GOLDEN = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'reference_suite_cases.json')))
+TARGETS = [t for t in GOLDEN if not t.startswith('_')]
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_TESTS), reason='reference checkout not present')
-@pytest.mark.parametrize('target,expr,n_expected', CPU_RUNNABLE, ids=[c[0] for c in CPU_RUNNABLE])
-def test_reference_tests_pass_unmodified(tmp_path, target, expr, n_expected):
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, 'compat'), ROOT]),
-               CUDA_VISIBLE_DEVICES='')
-    cmd = [sys.executable, '-m', 'pytest', '--import-mode=importlib', '-q', '-p', 'no:cacheprovider',
-           os.path.join(REFERENCE_TESTS, target)]
-    if expr:
-        cmd += ['-k', expr]
-    out = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=str(tmp_path), env=env)
-    tail = out.stdout[-3000:] + out.stderr[-1000:]
-    summary = re.search(r'(\d+) passed', out.stdout)
-    assert out.returncode == 0 and summary, tail
-    assert int(summary.group(1)) == n_expected and ' failed' not in out.stdout.splitlines()[-1], tail
+@pytest.mark.parametrize('target', TARGETS, ids=[t.replace('::', '-') for t in TARGETS])
+def test_reference_cases_pass_through_compat(tmp_path, target):
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, 'compat'), ROOT]), CUDA_VISIBLE_DEVICES='')
+    out = subprocess.run([sys.executable, '-m', 'tests.reference_cases', target], capture_output=True, text=True,
+                         timeout=900, cwd=str(tmp_path), env=env)
+    tail = out.stdout[-3000:] + out.stderr[-3000:]
+    passed = sorted(line.split(' ', 1)[1] for line in out.stdout.splitlines() if line.startswith('PASS '))
+    assert out.returncode == 0 and passed == GOLDEN[target], tail
